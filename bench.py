@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Mpixels/s of the feature-detection hot path on synthetic frames.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--workload W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--workload W] [--impl reference] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...        (one rank per GPU, frames sharded, no
                                                             data-path collective: weak scaling)
 
@@ -96,6 +96,25 @@ class ClockSampler:
         reasons = [n for i, n in enumerate(names) if any(len(r) > 2 + i and r[2 + i].lower().startswith("active") for r in rows)]
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None, "reasons": reasons,
                 "samples": len(sm)}
+
+
+DUMP_SAMPLE = 4 << 20      # elements kept of a larger output by --dump-outputs: <= 48 MB in all for every workload
+
+
+def dump_outputs(outdir, outputs):
+    """Writes {name: array} as outdir/<name>.npy in float32 (float32 and 8/16-bit integer outputs) or float64 (the
+    others): exact either way.  An array of more than DUMP_SAMPLE elements is replaced by a fixed seeded sample of its
+    rows (of its elements when 1-D), in their original order, so that two builds can be compared entry by entry."""
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in outputs.items():
+        a = np.asarray(a)
+        small = a.dtype == np.float32 or (a.dtype.kind in "iub" and a.dtype.itemsize <= 2)
+        a = a.astype(np.float32 if small else np.float64)
+        row = int(np.prod(a.shape[1:])) if a.ndim > 1 else 1
+        if a.size > DUMP_SAMPLE:
+            keep = np.sort(np.random.default_rng(0).choice(len(a), DUMP_SAMPLE // row, replace=False, shuffle=False))
+            a = a[keep]
+        np.save(os.path.join(outdir, name + ".npy"), a)
 
 
 def grey_of(rgb):
@@ -220,7 +239,13 @@ def main():
     ap.add_argument("--ref-frames", type=int, default=0, help="frames per reference step (0 = bounded by cores / memory / time)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-mode", action="store_true", help="device steps only (for ncu launch lists): no per-detector, e2e or CPU legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, float32/float64: Harris corner "
+                         "counts, raster indices y*nx+x and strengths; Canny edge maps and edge-pixel counts; FHOG features; "
+                         "SURF counts and point records; large arrays as a seeded sample (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -285,7 +310,7 @@ def main():
         surf_rec = torch.empty((B, SURF_KW["max_points"], 70), dtype=torch.float64).pin_memory().numpy()
     ev_fork = torch.cuda.Event()
     ctxs = [ctx] + ([ctx_c] if "canny" in dets else []) + ([ctx_f] if "fhog" in dets else [])
-    surf_counts = []
+    surf_counts, surf_last = [], {}
 
     def harris_dev(d_grey):
         # certified path: fused response + error bound -> tolerant NMS -> exact patches -> reference-identical lists
@@ -296,6 +321,7 @@ def main():
         if "surf" in dets:
             _, c = Dl.surf_dev(f["rgb"], B, NY, NX, rec=surf_rec, stream=sp, **SURF_KW)
             surf_counts[:] = [int(c.mean())]
+            surf_last["counts"] = c
             return
         ev_fork.record(stream)
         if "canny" in dets:
@@ -346,6 +372,16 @@ def main():
     ms_total = timed(step_dev, K)
     t_region1 = time.perf_counter()
     launches = launch_total() - l0
+    snap = {}                                # the last timed step's outputs, before anything below overwrites them
+    if args.dump_outputs and rank == 0:
+        if "surf" in dets:
+            snap.update(surf_records=surf_rec.copy(), surf_counts=surf_last["counts"].copy())
+        if "harris" in dets:
+            snap.update(harris_counts=d_cnt.clone(), harris_xy=d_xy.clone(), harris_strength=d_st.clone())
+        if "canny" in dets:
+            snap.update(canny_edges=d_edges.clone(), canny_nonzero=d_nz.clone())
+        if "fhog" in dets:
+            snap.update(fhog=d_hog.clone())
     clocks = None
     if rank == 0:
         note = "timed region"
@@ -360,6 +396,19 @@ def main():
             note = "timed region + untimed continuation of the same steps (region shorter than the 100 ms sampling period)"
         clocks = sampler.stop(t_region0, t_region1)
         clocks["window"] = note
+    if snap:
+        out = {k: v.cpu().numpy() if torch.is_tensor(v) else v for k, v in snap.items()}
+        if "harris_counts" in out:          # the stored part of each frame's corner list, frame after frame
+            n = np.minimum(out["harris_counts"], cap)
+            for k in ("harris_xy", "harris_strength"):
+                out[k] = np.concatenate([out[k][i, :n[i]] for i in range(B)])
+        if "surf_counts" in out:
+            out["surf_records"] = np.concatenate([out["surf_records"][i, :c] for i, c in enumerate(out["surf_counts"])])
+        for k in ("canny_edges", "fhog"):
+            if k in out:
+                out[k] = out[k].reshape(-1)
+        dump_outputs(args.dump_outputs, out)
+        del snap, out
     ms_step = ms_total / K
     value = world * B * NX * NY / (ms_step * 1e-3) / 1e6
 

@@ -3,16 +3,35 @@
 `orc`  : oracle/liboracle.so      the C restatement in oracle/*_oracle.c (always buildable)
 `ref`  : oracle/_ref/libref_*.so  the UNMODIFIED reference compiled in place from /root/reference
                                    (present where it was built; travels to the GPU box as a .so)
+Tests compare with the reference through outputs frozen under tests/golden/ (whole arrays or their
+`digest`s), so they need no `ref` library at run time; the tests/golden/make_golden*.py scripts use it.
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may
 import this module.  The product package image_b200 never does.
 """
 import ctypes as C
+import hashlib
 import os
 import subprocess
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+
+
+def digest(a):
+    """'<dtype>[shape]:sha256' of an array's values.  Two arrays of one dtype have equal digests exactly when
+    np.array_equal holds (-0.0 and +0.0 hash alike; a NaN fails, as it fails array_equal), so a stored digest
+    of a reference output keeps a bit-exact comparison without storing the output."""
+    a = np.ascontiguousarray(a)
+    if a.dtype.kind == "f":
+        assert not np.isnan(a).any(), "NaN in an array to be compared"
+        a = a + a.dtype.type(0)                       # -0.0 -> +0.0
+    return "%s%s:%s" % (a.dtype.str, list(a.shape), hashlib.sha256(a.tobytes()).hexdigest())
+
+
+def digests(**values):
+    """{name: digest(array) or int(scalar)}: one entry of tests/golden/reference_digests.json."""
+    return {k: digest(v) if isinstance(v, np.ndarray) else int(v) for k, v in values.items()}
 
 
 def build(ref=True):

@@ -31,3 +31,12 @@ def golden():
     def load(name):
         return np.load(os.path.join(gdir, name + ".npz"))
     return load
+
+
+@pytest.fixture(scope="session")
+def reference_digests():
+    """Outputs of the unmodified reference on the parity tests' own inputs, as oracle.digests() entries
+    (written by tests/golden/make_golden_parity.py)."""
+    import json
+    with open(os.path.join(ROOT, "tests", "golden", "reference_digests.json")) as f:
+        return json.load(f)

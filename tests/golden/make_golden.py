@@ -58,7 +58,7 @@ def harris_cases(img_yx, tag):
         out[name + "_x"], out[name + "_y"], out[name + "_s"] = x, y, s
         out[name + "_args"] = np.array(repr(kw))
     R, _ = po.harris_response(img_yx, impl="ref")
-    out["R_default"] = R
+    out["R_default_digest"] = np.array(po.digest(R))      # the float32 plane itself does not compress (1 MB)
     np.savez_compressed(os.path.join(OUT, "harris_%s.npz" % tag), **out)
     print("harris", tag, {k: len(out[k + "_x"]) for k in cases})
 

@@ -48,7 +48,7 @@ def boat():
     img = np.asarray(Image.open(REF + "/image.dlib/inst/extdata/cruise_boat.png").convert("RGB"))
     f = {"image": img}
     for name, kw in {"default": dict(cell=8, frp=1, fcp=1), "cell4_pad3": dict(cell=4, frp=3, fcp=3)}.items():
-        f[name] = po.fhog(img, impl="ref", **kw).astype(np.float32)
+        f[name + "_digest"] = np.array(po.digest(po.fhog(img, impl="ref", **kw).astype(np.float32)))   # 0.4 / 1.3 MB as arrays
         f[name + "_args"] = np.array(repr(kw))
     np.savez_compressed(os.path.join(OUT, "fhog_boat.npz"), **f)
     # cell_size == 1 (dlib's separate routine): a 96 x 128 crop keeps the fixture small (31 floats per pixel)

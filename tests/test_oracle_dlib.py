@@ -1,5 +1,5 @@
-"""CPU tests: FHOG / SURF restatements against dlib's own golden vectors, the frozen outputs of the
-unmodified reference on its fixture, and (when present) the in-place reference build oracle/_ref."""
+"""CPU tests: FHOG / SURF restatements against dlib's own golden vectors and the frozen outputs of the
+unmodified reference on its fixture and on synthetic frames."""
 import ast
 
 import numpy as np
@@ -21,7 +21,7 @@ def test_fhog_oracle_matches_reference_on_fixture(oracle, golden, case):
     g = golden("fhog_boat")
     kw = ast.literal_eval(str(g[case + "_args"]))
     hog = oracle.fhog(g["image"], **kw)
-    assert np.array_equal(hog.astype(np.float32), g[case])          # bit-exact (outputs are floats)
+    assert oracle.digest(hog.astype(np.float32)) == str(g[case + "_digest"])          # bit-exact (outputs are floats)
 
 
 @pytest.mark.parametrize("case", ["default", "all"])
@@ -45,31 +45,45 @@ def test_integral_image_property(oracle):
     assert np.array_equal(sat, grey.cumsum(0).cumsum(1))
 
 
-def _need_ref(oracle):
-    if not oracle.have_ref("dlib"):
-        pytest.skip("oracle/_ref/libref_dlib.so not built (no /root/reference here)")
+# The reference's outputs on the synthetic inputs below are frozen in tests/golden/reference_digests.json
+# (make_golden_parity.py runs it).
 
-
-def test_fhog_oracle_equals_reference_incl_colour_ties(oracle):
-    _need_ref(oracle)
+def fhog_frame_cases():
+    """(key, image, cell, frp, fcp)."""
     from image_b200 import synth
     rng = np.random.default_rng(1)
     for rows, cols, cell, frp, fcp in [(100, 131, 8, 1, 1), (97, 203, 4, 1, 1), (120, 160, 8, 2, 5), (75, 90, 5, 1, 1), (23, 300, 8, 1, 1)]:
-        for im in (synth.frame_rgb(rows, rows, cols), (synth.frame_rgb(cols, rows, cols) // 16 * 16).astype(np.uint8),
-                   rng.integers(0, 255, (rows, cols, 3)).astype(np.uint8)):
-            a, b = oracle.fhog(im, cell, frp, fcp, impl="ref"), oracle.fhog(im, cell, frp, fcp)
-            assert a.shape == b.shape and np.array_equal(a, b)
+        for j, im in enumerate((synth.frame_rgb(rows, rows, cols), (synth.frame_rgb(cols, rows, cols) // 16 * 16).astype(np.uint8),
+                                rng.integers(0, 255, (rows, cols, 3)).astype(np.uint8))):
+            yield "fhog_frame_%dx%d_cell%d_pad%d_%d_%d" % (rows, cols, cell, frp, fcp, j), im, cell, frp, fcp
 
 
-def test_surf_oracle_equals_reference(oracle):
-    _need_ref(oracle)
+def surf_frame_cases():
+    """(key, image, max_points, threshold)."""
     from image_b200 import synth
     for rows, cols, mp, thr in [(300, 417, 10000, 10.0), (480, 640, 50, 30.0), (540, 960, 10000, 30.0)]:
-        img = synth.frame_blobs(rows + cols, rows, cols)
-        a, b = oracle.surf(img, mp, thr, impl="ref"), oracle.surf(img, mp, thr)
-        assert len(a["x"]) == len(b["x"])
-        for k in a:
-            assert np.array_equal(a[k], b[k]), k
+        yield "surf_frame_%dx%d_%d_%g" % (rows, cols, mp, thr), synth.frame_blobs(rows + cols, rows, cols), mp, thr
+
+
+def otsu_cases():
+    """(key, pixels, width, height, threshold)."""
+    rng = np.random.default_rng(5)
+    for k in range(12):
+        hh, ww = int(rng.integers(1, 60)), int(rng.integers(1, 80))
+        x = rng.integers(0, 256, hh * ww).astype(np.float64) if k % 2 else rng.random(hh * ww) * 255.9
+        for thr in (0, 33):
+            yield "otsu_%d_thr%d" % (k, thr), x, ww, hh, thr
+
+
+def test_fhog_oracle_equals_reference_incl_colour_ties(oracle, reference_digests):
+    for key, im, cell, frp, fcp in fhog_frame_cases():
+        assert oracle.digests(fhog=oracle.fhog(im, cell, frp, fcp)) == reference_digests[key], key
+
+
+def test_surf_oracle_equals_reference(oracle, reference_digests):
+    for key, img, mp, thr in surf_frame_cases():
+        b = oracle.surf(img, mp, thr)
+        assert oracle.digests(points=len(b["x"]), **b) == reference_digests[key], key
 
 
 def test_fhog_cell_size_1_oracle_matches_reference_fixture(oracle, golden):
@@ -80,20 +94,15 @@ def test_fhog_cell_size_1_oracle_matches_reference_fixture(oracle, golden):
     assert int((out != 0).sum()) <= 6 * out.shape[0] * out.shape[1]
 
 
-def test_otsu_oracle_matches_reference_build_and_fixture(oracle, golden):
-    """image.Otsu (8f rank 4): the restatement equals the unmodified source compiled in place, and the
-    frozen output of that build on the package's own coins.jpeg."""
+def test_otsu_oracle_matches_reference_build_and_fixture(oracle, golden, reference_digests):
+    """image.Otsu (8f rank 4): the restatement equals the unmodified source compiled in place on random
+    inputs, and the frozen output of that build on the package's own coins.jpeg."""
     g = golden("otsu_coins")
     img = g["image"].astype(np.float64)
     h, w = img.shape
     o, t = oracle.otsu(img.ravel(order="F"), w, h, 0)
     assert t == int(g["threshold"])
     assert np.array_equal(o.reshape(img.shape, order="F") > 0, np.unpackbits(g["mask"])[: img.size].reshape(img.shape).astype(bool))
-    if oracle.have_ref("otsu"):
-        rng = np.random.default_rng(5)
-        for k in range(12):
-            hh, ww = int(rng.integers(1, 60)), int(rng.integers(1, 80))
-            x = rng.integers(0, 256, hh * ww).astype(np.float64) if k % 2 else rng.random(hh * ww) * 255.9
-            for thr in (0, 33):
-                a, b = oracle.otsu(x, ww, hh, thr), oracle.otsu(x, ww, hh, thr, impl="ref")
-                assert a[1] == b[1] and np.array_equal(a[0], b[0])
+    for key, x, ww, hh, thr in otsu_cases():
+        a, ta = oracle.otsu(x, ww, hh, thr)
+        assert oracle.digests(out=a, threshold=ta) == reference_digests[key], key

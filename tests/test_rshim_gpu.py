@@ -88,19 +88,24 @@ def test_otsu_shim(shim, oracle):
     assert t == ot and np.array_equal(out, o)
 
 
-def test_contour_front_shim_feeds_the_reference_chainer(shim, oracle):
+CONTOUR_SHIM_FRAME = (24, 150, 230)                                  # (seed, Y, X)
+
+
+def test_contour_front_shim_feeds_the_reference_chainer(shim, oracle, reference_digests):
     """b2f_contour_front (rshim/contour_front.c) rebuilds the planes the reference's sequential chainer reads: Ex / Ey equal
-    the reference's planes everywhere, Gx / Gy at every edge point, and the reference's own chain_edge_points ->
-    simplify_chains -> list_chained_edge_points run on them gives the same curves as on the reference's planes."""
+    the reference's planes everywhere, Gx / Gy at every edge point (the only pixels where its chain() reads them), so the
+    reference's own chain_edge_points -> simplify_chains -> list_chained_edge_points gives the same curves on them as on
+    the reference's planes; where the reference is built, that is checked by running it."""
     from image_b200 import synth
-    Y, X = 150, 230
-    img = synth.frame_shapes(24, Y, X).astype(np.float64)
+    seed, Y, X = CONTOUR_SHIM_FRAME
+    img = synth.frame_shapes(seed, Y, X).astype(np.float64)
     gauss = np.zeros((Y, X)); Gx = np.zeros((Y, X)); Gy = np.zeros((Y, X)); Ex = np.zeros((Y, X)); Ey = np.zeros((Y, X))
     shim.b2f_contour_front.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_double] + [C.c_void_p] * 5
     assert shim.b2f_contour_front(_p(img), X, Y, 0.0, _p(gauss), _p(Gx), _p(Gy), _p(Ex), _p(Ey)) == 0
     g = oracle.contour_gaussian(img)
     assert np.array_equal(gauss, g)
     r = oracle.contour_edge_points(g)
+    assert oracle.digests(**r) == reference_digests["contour_shim_frame"]    # the reference's edge points and gradients
     ex = np.full(X * Y, -1.0); ey = np.full(X * Y, -1.0)
     ex[r["idx"]] = r["Ex"]; ey[r["idx"]] = r["Ey"]
     assert np.array_equal(Ex.ravel(), ex) and np.array_equal(Ey.ravel(), ey)
